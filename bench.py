@@ -29,6 +29,13 @@ weights (seed 3407).  Every step uses a fresh slice of the corpus; the per-step 
          200k-premise corpus: encode of one state + access bitmask + top-k + Premise objects.
   sweep (N = 1)  BASELINE configs[4]: encoder throughput at seq_len {128,512,1024,2048} x batch {32,128,512}.
   reindex_2048 (N = 1)  the shape retrieval/index.py:33 indexes at: max_seq_len 2048, token length ~ U[17, 2048].
+
+`--dump-outputs DIR` writes what rank 0's timed calls returned in their last repetition, so that two builds
+run with the same arguments (hence the same seeded inputs) can be compared output for output:
+  reindex_embeddings.npy   float32 [rows, 1472], the last timed step's premise embeddings (bf16 widened); when a
+                           step holds more than 8192 premises, 8192 of them, the same seeded sample every run,
+                           and reindex_rows.npy (float64) says which
+  retrieve_q{1024,64,1}_indices.npy / _scores.npy   float64 [Q, 100], the global top-k rows and their fp64 scores
 """
 from __future__ import annotations
 
@@ -37,6 +44,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import time
 from pathlib import Path
 
@@ -51,6 +59,8 @@ from reprover_b200 import synth  # noqa: E402
 D_MODEL = 1472
 N_CORPUS = 200_000
 MAX_SEQ_LEN = 512
+# 8192 x 1472 fp32 = 48 MB: with the retrieve results a dump stays under 64 MB
+DUMP_MAX_ROWS = 8192
 
 
 def cpu_threads() -> int:
@@ -211,6 +221,13 @@ def run_engine(args) -> dict:
     ms_dev = max_over_ranks(e0.elapsed_time(e1), world, dev)
     prof = eng.read_profile()
     eng.set_profiling(False)
+    dump = {} if args.dump_outputs and rank == 0 else None
+    if dump is not None:
+        rows = np.arange(P)
+        if P > DUMP_MAX_ROWS:
+            rows = np.sort(np.random.default_rng(synth.SEED).choice(P, DUMP_MAX_ROWS, replace=False))
+            dump["reindex_rows"] = rows.astype(np.float64)
+        dump["reindex_embeddings"] = out[torch.from_numpy(rows).to(dev)].float().cpu().numpy()
     timed_tokens = sum(int(tok_lens[lo:hi].sum()) for lo, hi in step_slices[W:W + K])
     timed_flops = sum(encoder_flops(tok_lens[lo:hi]) for lo, hi in step_slices[W:W + K])
     value = world * P * K / (ms_dev / 1e3)
@@ -277,9 +294,9 @@ def run_engine(args) -> dict:
         E = synth.random_unit_rows(n_idx, D_MODEL, 1000 + rank, dev)
         handle = IndexHandle(E)
         Q_all = synth.random_unit_rows(1024, D_MODEL, 999, dev)   # same queries on every rank
-        retrieve = retrieve_leg(Q_all, E, handle, k, rank, world, dev, peaks, e0, e1, K, W, check_parity=True)
-        retrieve_q64 = retrieve_leg(Q_all[:64].contiguous(), E, handle, k, rank, world, dev, peaks, e0, e1, K, W)
-        retrieve_q1 = retrieve_leg(Q_all[:1].contiguous(), E, handle, k, rank, world, dev, peaks, e0, e1, K, W)
+        retrieve = retrieve_leg(Q_all, E, handle, k, rank, world, dev, peaks, e0, e1, K, W, check_parity=True, dump=dump)
+        retrieve_q64 = retrieve_leg(Q_all[:64].contiguous(), E, handle, k, rank, world, dev, peaks, e0, e1, K, W, dump=dump)
+        retrieve_q1 = retrieve_leg(Q_all[:1].contiguous(), E, handle, k, rank, world, dev, peaks, e0, e1, K, W, dump=dump)
         retrieve["guard"] = handle.stats()
         if rank == 0 and world == 1 and not args.skip_cpu_baseline:
             retrieve["cpu_baseline"] = cpu_baseline_retrieve(E, Q_all, k)
@@ -315,6 +332,10 @@ def run_engine(args) -> dict:
         "retrieve_q1": retrieve_q1, "retrieve_q64": retrieve_q64, "retrieve_single": retrieve_single,
         "sweep": sweep, "reindex_2048": reindex_2048,
     }
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), arr)
     parity = (retrieve or {}).get("parity")
     if parity is not None and parity["mismatches"] != 0:
         exc = SystemExit(f"[bench] retrieve parity FAILED: {parity}")
@@ -366,7 +387,7 @@ def brute_force_parity(Q, E, k, rank, world, dev, got_idx, got_s64, n_sample=64)
     return out
 
 
-def retrieve_leg(Q, E, handle, k, rank, world, dev, peaks, e0, e1, K, W, check_parity=False):
+def retrieve_leg(Q, E, handle, k, rank, world, dev, peaks, e0, e1, K, W, check_parity=False, dump=None):
     from reprover_b200.dist import sharded_topk
     from reprover_b200.retrieval_ops import sim_topk
 
@@ -387,10 +408,13 @@ def retrieve_leg(Q, E, handle, k, rank, world, dev, peaks, e0, e1, K, W, check_p
     barrier(world)
     e0.record()
     for _ in range(reps):
-        retrieve_dev()
+        last = retrieve_dev()
     e1.record()
     barrier(world)
     ms_r = max_over_ranks(e0.elapsed_time(e1), world, dev) / reps
+    if dump is not None:
+        dump[f"retrieve_q{nq}_indices"] = last[1].double().cpu().numpy()
+        dump[f"retrieve_q{nq}_scores"] = last[3].cpu().numpy()
     # e2e: queries from pinned host memory, results back to the host
     res_scores = torch.empty(nq, k, dtype=torch.float32).pin_memory()
     res_idx = torch.empty(nq, k, dtype=torch.int64).pin_memory()
@@ -653,8 +677,12 @@ def main():
     ap.add_argument("--skip-retrieve", action="store_true")
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--skip-extras", action="store_true", help="skip retrieve_single / sweep / reindex_2048 (N = 1 legs)")
-    ap.add_argument("--tmp", default="/tmp/rpx_bench")
+    ap.add_argument("--tmp", default=None,
+                    help="where the e2e leg's checkpoint goes, in a fresh directory removed at exit (default: the system's temp dir)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed calls' last outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "engine":
+        ap.error("--dump-outputs applies to the engine arm")
     if args.impl == "engine" and args.warmup < 3:
         print(f"[bench] --warmup {args.warmup} raised to 3 (timing rules: at least 3 warm-up steps)", file=sys.stderr)
         args.warmup = 3
@@ -664,7 +692,9 @@ def main():
     real_stdout = os.dup(1)
     os.dup2(2, 1)
     try:
-        res = run_reference(args) if args.impl == "reference" else run_engine(args)
+        with tempfile.TemporaryDirectory(prefix="rpx_bench_", dir=args.tmp) as tmp:
+            args.tmp = tmp
+            res = run_reference(args) if args.impl == "reference" else run_engine(args)
     except SystemExit as exc:
         res = getattr(exc, "bench_result", None)
         if res is not None:

@@ -1,8 +1,9 @@
 """Dry run of tests/test_zz_reference_golden_gpu.py on the CPU: the CUDA engine is replaced by the HF oracle
 (bf16-rounded outputs, CPU tensors), the device top-k by the C oracle.  Validates the test logic only."""
 import json, sys, types
+from pathlib import Path
 import numpy as np, torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
 from oracle import reference_path as ref, c_oracle
 from reprover_b200 import synth, dist as rdist, retrieval_ops
 from reprover_b200.retriever import B200PremiseRetriever
