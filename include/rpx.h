@@ -149,8 +149,10 @@ int32_t rpx_t5_relative_bucket(int32_t relative_position, int32_t num_buckets, i
 
 /* Debug / parity hook: when non-NULL, every encode call also writes the fp32
  * residual stream after the embedding and after each block to
- * d_hidden[(layer) * n_tokens * d_model ...] (num_layers + 1 slabs, packed tokens). */
-int rpx_encoder_set_debug_hidden(rpx_encoder* enc, float* d_hidden);
+ * d_hidden[(slab * max_tokens + t) * d_model ...] (num_layers + 1 slabs of max_tokens rows;
+ * the call's packed tokens fill the first T rows of each).  An encode call with more than
+ * `max_tokens` packed tokens returns RPX_ERR_WORKSPACE while the hook is set. */
+int rpx_encoder_set_debug_hidden(rpx_encoder* enc, float* d_hidden, int64_t max_tokens);
 
 /* Per-kernel-class device timing (CUDA events on the launch stream).  Classes:
  * 0 embed, 1 qkv gemm, 2 attention, 3 o-proj gemm, 4 ffn-up gemm, 5 ffn-down gemm, 6 pool. */
@@ -249,6 +251,20 @@ int rpx_gemm_bf16_f32(const void* d_A, const void* d_B, float* d_C, int32_t M, i
 /* Same contract through the 2-CTA (cta_group::2, 256 x 256 tile) form of the core. */
 int rpx_gemm2_bf16_f32(const void* d_A, const void* d_B, float* d_C, int32_t M, int32_t N,
                        int32_t K, void* stream);
+
+/*
+ * The encoder's T5 self-attention on caller-provided operands, for parity tests of the kernels:
+ *   d_qkv        [T, 3 * n_heads * 64] bf16 packed tokens, q | k | v (head h at columns h*64 of each third)
+ *   d_out        [T, n_heads * 64] bf16; rows [cu[s], cu[s+1]) of each sequence are written, no others
+ *   d_cu_seqlens / h_cu_seqlens  the same n_seqs + 1 token offsets on the device and on the host;
+ *                cu[0] = 0, every sequence non-empty, T = cu[n_seqs]
+ *   d_bias_lut   [n_heads][2 * rel_max_distance + 1] fp32, entry clamp(key - query, +-R) + R
+ *   kernel       0 = throughput kernel (any length), 1 = latency kernel (RPX_ERR_UNSUPPORTED when a
+ *                sequence is longer than 1024 tokens or the bias table does not fit its shared memory)
+ * out = softmax(q k^T + bias) v per sequence and head (no 1/sqrt(d) scaling, as in T5). */
+int rpx_t5_attention_bf16(const void* d_qkv, void* d_out, const int32_t* d_cu_seqlens,
+                          const int32_t* h_cu_seqlens, int32_t n_seqs, int32_t n_heads,
+                          const float* d_bias_lut, int32_t rel_max_distance, int32_t kernel, void* stream);
 
 #ifdef __cplusplus
 }

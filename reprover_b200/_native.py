@@ -88,7 +88,7 @@ _SIGNATURES = {
                                  C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]),
     "rpx_encoder_set_latency_tokens": (C.c_int, [C.c_void_p, C.c_int32]),
     "rpx_t5_relative_bucket": (C.c_int32, [C.c_int32, C.c_int32, C.c_int32]),
-    "rpx_encoder_set_debug_hidden": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "rpx_encoder_set_debug_hidden": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64]),
     "rpx_encoder_set_profiling": (C.c_int, [C.c_void_p, C.c_int32]),
     "rpx_encoder_read_profile": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_int64)]),
     "rpx_index_state_bytes": (C.c_size_t, []),
@@ -113,6 +113,8 @@ _SIGNATURES = {
                                     C.c_void_p]),
     "rpx_gemm2_bf16_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                      C.c_void_p]),
+    "rpx_t5_attention_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32), C.c_int32,
+                                        C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

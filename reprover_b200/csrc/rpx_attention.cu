@@ -645,9 +645,13 @@ t5_attention_short_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid
 
 }  // namespace
 
+bool t5_attention_bias_fits(int max_distance) {
+  return 1024 + kAttnSmemFixed + (size_t)4 * bias_copy_stride(max_distance) * 4 + 128 <= 100 * 1024;
+}
+
 int launch_t5_attention(const __nv_bfloat16* qkv, __nv_bfloat16* out, const int32_t* cu_seqlens,
                         const float* bias_lut, int n_tokens, int n_seqs, int max_len, int n_heads, int d_kv,
-                        int max_distance, cudaStream_t stream, bool latency) {
+                        int max_distance, cudaStream_t stream, AttnKernel kernel) {
   RPX_REQUIRE(d_kv == kHD, RPX_ERR_UNSUPPORTED, "attention: d_kv=%d (only 64 is implemented)", d_kv);
   RPX_REQUIRE(n_seqs > 0 && max_len > 0 && n_tokens > 0, RPX_ERR_INVALID, "attention: empty batch");
   RPX_REQUIRE(n_seqs <= 65535 && n_heads <= 65535, RPX_ERR_UNSUPPORTED, "attention: grid limits exceeded");
@@ -656,9 +660,13 @@ int launch_t5_attention(const __nv_bfloat16* qkv, __nv_bfloat16* out, const int3
   RPX_TRY(get_device_info(&dev));
   CUtensorMap tm_q, tm_kv;
   RPX_TRY(make_tmap_bf16_2d(&tm_kv, qkv, (uint64_t)n_tokens, (uint64_t)3 * inner, (uint64_t)3 * inner, kKT));
-  if (latency && max_len <= kShortMaxKeys) {
+  if (kernel != AttnKernel::Throughput) {
     const size_t smem_short = 1024 + kShortOffBias + (size_t)4 * bias_copy_stride(max_distance) * 4 + 128;
-    if (smem_short <= dev.smem_optin) {
+    const bool short_ok = max_len <= kShortMaxKeys && smem_short <= dev.smem_optin;
+    RPX_REQUIRE(short_ok || kernel == AttnKernel::Auto, RPX_ERR_UNSUPPORTED,
+                "attention: the latency kernel takes at most %d keys and a bias table within %zu B of shared memory "
+                "(max_len=%d, %zu B)", kShortMaxKeys, dev.smem_optin, max_len, smem_short);
+    if (short_ok) {
       RPX_TRY(make_tmap_bf16_2d(&tm_q, qkv, (uint64_t)n_tokens, (uint64_t)3 * inner, (uint64_t)3 * inner, kShortQ));
       static thread_local int configured_short = -1;
       if (configured_short != dev.device) {
@@ -674,7 +682,8 @@ int launch_t5_attention(const __nv_bfloat16* qkv, __nv_bfloat16* out, const int3
   }
   RPX_TRY(make_tmap_bf16_2d(&tm_q, qkv, (uint64_t)n_tokens, (uint64_t)3 * inner, (uint64_t)3 * inner, kQT));
   const size_t smem = 1024 + kAttnSmemFixed + (size_t)4 * bias_copy_stride(max_distance) * 4 + 128;
-  RPX_REQUIRE(smem <= 100 * 1024, RPX_ERR_UNSUPPORTED, "attention: bias table too large (%zu B of shared memory)", smem);
+  RPX_REQUIRE(t5_attention_bias_fits(max_distance), RPX_ERR_UNSUPPORTED,
+              "attention: bias table too large (%zu B of shared memory)", smem);
   static thread_local int configured = -1;
   if (configured != dev.device) {
     RPX_CUDA_OK(cudaFuncSetAttribute(t5_attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
@@ -687,3 +696,25 @@ int launch_t5_attention(const __nv_bfloat16* qkv, __nv_bfloat16* out, const int3
 }
 
 }  // namespace rpx
+
+extern "C" int rpx_t5_attention_bf16(const void* d_qkv, void* d_out, const int32_t* d_cu_seqlens,
+                                     const int32_t* h_cu_seqlens, int32_t n_seqs, int32_t n_heads,
+                                     const float* d_bias_lut, int32_t rel_max_distance, int32_t kernel, void* stream) {
+  using namespace rpx;
+  RPX_REQUIRE(d_qkv && d_out && d_cu_seqlens && h_cu_seqlens && d_bias_lut, RPX_ERR_INVALID,
+              "rpx_t5_attention_bf16: null pointer");
+  RPX_REQUIRE(n_seqs > 0 && n_heads > 0 && rel_max_distance > 0, RPX_ERR_INVALID,
+              "rpx_t5_attention_bf16: n_seqs=%d n_heads=%d rel_max_distance=%d", n_seqs, n_heads, rel_max_distance);
+  RPX_REQUIRE(kernel == 0 || kernel == 1, RPX_ERR_INVALID, "rpx_t5_attention_bf16: kernel=%d (0 or 1)", kernel);
+  // the grid and the tensor maps are sized from the host copy: every sequence must lie inside [0, T)
+  RPX_REQUIRE(h_cu_seqlens[0] == 0, RPX_ERR_INVALID, "rpx_t5_attention_bf16: cu_seqlens[0]=%d", h_cu_seqlens[0]);
+  int max_len = 0;
+  for (int s = 0; s < n_seqs; ++s) {
+    const int len = h_cu_seqlens[s + 1] - h_cu_seqlens[s];
+    RPX_REQUIRE(len > 0, RPX_ERR_INVALID, "rpx_t5_attention_bf16: sequence %d has length %d", s, len);
+    if (len > max_len) max_len = len;
+  }
+  return launch_t5_attention(static_cast<const __nv_bfloat16*>(d_qkv), static_cast<__nv_bfloat16*>(d_out), d_cu_seqlens,
+                             d_bias_lut, h_cu_seqlens[n_seqs], n_seqs, max_len, n_heads, 64, rel_max_distance,
+                             static_cast<cudaStream_t>(stream), kernel == 0 ? AttnKernel::Throughput : AttnKernel::Latency);
+}

@@ -149,6 +149,7 @@ struct rpx_encoder {
   const float* bias_lut = nullptr;
   std::vector<rpx::LayerW> layers;
   float* debug_hidden = nullptr;
+  int64_t debug_tokens = 0;  // capacity of debug_hidden in tokens (the slab stride)
   bool profiling = false;
   std::vector<rpx::ProfRec> prof_pending;
   std::vector<cudaEvent_t> event_pool;
@@ -206,6 +207,9 @@ int validate_cfg(const rpx_t5_config* c) {
                   c->rel_max_distance <= 2048,
               RPX_ERR_UNSUPPORTED, "unsupported relative attention config (%d buckets, max distance %d)",
               c->rel_buckets, c->rel_max_distance);
+  RPX_REQUIRE(t5_attention_bias_fits(c->rel_max_distance), RPX_ERR_UNSUPPORTED,
+              "rel_max_distance=%d: the attention kernel's shared memory does not hold that bias table",
+              c->rel_max_distance);
   return RPX_OK;
 }
 
@@ -335,7 +339,7 @@ int forward_latency_layer(rpx_encoder* e, const Workspace& ws, const LayerW& w, 
   {
     Prof p(e, st, 2);
     RPX_TRY(launch_t5_attention(ws.qkv, ws.attn, ws.cu_tokens, e->bias_lut, T, S, max_len, c.num_heads, c.d_kv,
-                                c.rel_max_distance, st, true));
+                                c.rel_max_distance, st, AttnKernel::Auto));
   }
   {
     Prof p(e, st, 3);
@@ -380,6 +384,8 @@ int forward(rpx_encoder* e, const Workspace& ws, int T, int S, int max_len, void
   const bool latency = T <= e->latency_tokens && D % 32 == 0 && (3 * inner) % 32 == 0;
   const int P = latency ? e->n_parts_lat : e->n_parts;
   const float inv_d = 1.0f / (float)D;
+  RPX_REQUIRE(!e->debug_hidden || T <= e->debug_tokens, RPX_ERR_WORKSPACE,
+              "debug hidden-state buffer holds %lld tokens, the call has %d", (long long)e->debug_tokens, T);
   struct PdlScope {
     explicit PdlScope(bool on) { set_pdl_scope(on); }
     ~PdlScope() { set_pdl_scope(false); }
@@ -390,7 +396,7 @@ int forward(rpx_encoder* e, const Workspace& ws, int T, int S, int max_len, void
   }
   auto dump = [&](int slab) -> int {
     if (e->debug_hidden)
-      RPX_CUDA_OK(cudaMemcpyAsync(e->debug_hidden + (size_t)slab * T * D, ws.h32, (size_t)T * D * 4,
+      RPX_CUDA_OK(cudaMemcpyAsync(e->debug_hidden + (size_t)slab * e->debug_tokens * D, ws.h32, (size_t)T * D * 4,
                                   cudaMemcpyDeviceToDevice, st));
     return RPX_OK;
   };
@@ -414,7 +420,7 @@ int forward(rpx_encoder* e, const Workspace& ws, int T, int S, int max_len, void
     {
       Prof p(e, st, 2);
       RPX_TRY(launch_t5_attention(ws.qkv, ws.attn, ws.cu_tokens, e->bias_lut, T, S, max_len, c.num_heads, c.d_kv,
-                                  c.rel_max_distance, st));
+                                  c.rel_max_distance, st, AttnKernel::Throughput));
     }
     {
       Prof p(e, st, 3);
@@ -636,9 +642,12 @@ int rpx_encoder_set_latency_tokens(rpx_encoder* enc, int32_t max_tokens) {
   return RPX_OK;
 }
 
-int rpx_encoder_set_debug_hidden(rpx_encoder* enc, float* d_hidden) {
+int rpx_encoder_set_debug_hidden(rpx_encoder* enc, float* d_hidden, int64_t max_tokens) {
   RPX_REQUIRE(enc, RPX_ERR_INVALID, "null encoder");
+  RPX_REQUIRE(!d_hidden || max_tokens > 0, RPX_ERR_INVALID, "rpx_encoder_set_debug_hidden: max_tokens=%lld",
+              (long long)max_tokens);
   enc->debug_hidden = d_hidden;
+  enc->debug_tokens = d_hidden ? max_tokens : 0;
   return RPX_OK;
 }
 

@@ -10,9 +10,15 @@ namespace rpx {
 // ---- rpx_attention.cu
 // qkv [T, 3*heads*d_kv] bf16 packed tokens; out [T, heads*d_kv] bf16;
 // bias_lut [heads][2*max_distance+1] fp32, entry (delta + max_distance), delta = key - query clamped.
+// Throughput: t5_attention_tc_kernel (128-query CTAs, any length).  Latency: t5_attention_short_kernel
+// (32-query CTAs, max_len <= 1024, bias table within the shared-memory opt-in), RPX_ERR_UNSUPPORTED outside
+// that range.  Auto: the latency kernel where it can run, the throughput kernel otherwise.
+enum class AttnKernel { Throughput, Latency, Auto };
 int launch_t5_attention(const __nv_bfloat16* qkv, __nv_bfloat16* out, const int32_t* cu_seqlens,
                         const float* bias_lut, int n_tokens, int n_seqs, int max_len, int n_heads, int d_kv,
-                        int max_distance, cudaStream_t stream, bool latency = false);
+                        int max_distance, cudaStream_t stream, AttnKernel kernel);
+// Whether the throughput kernel (the one every length can use) holds the bias table of `max_distance`.
+bool t5_attention_bias_fits(int max_distance);
 
 // ---- rpx_elementwise.cu
 // ByT5 tokenisation of packed byte strings into packed token ids (byte + 3, EOS = 1 last,

@@ -299,14 +299,16 @@ class T5EncoderEngine:
 
     # ------------------------------------------------------------------ debug / profiling
     def set_debug_hidden(self, n_tokens: Optional[int]) -> Optional[torch.Tensor]:
-        """Allocate (or drop, with None) the [layers+1, n_tokens, d_model] fp32 hidden-state dump."""
+        """Allocate (or drop, with None) the [layers+1, n_tokens, d_model] fp32 hidden-state dump.  Each
+        engine call then writes its T packed tokens to rows [0, T) of every slab; a call with more than
+        `n_tokens` tokens fails with RPX_ERR_WORKSPACE."""
         if n_tokens is None:
+            _native.check(self.lib.rpx_encoder_set_debug_hidden(self._handle, None, 0))
             self._debug_buf = None
-            _native.check(self.lib.rpx_encoder_set_debug_hidden(self._handle, None))
             return None
         self._debug_buf = torch.zeros(self._cfg.num_layers + 1, n_tokens, self.hidden_size, dtype=torch.float32,
                                       device=self.device)
-        _native.check(self.lib.rpx_encoder_set_debug_hidden(self._handle, self._debug_buf.data_ptr()))
+        _native.check(self.lib.rpx_encoder_set_debug_hidden(self._handle, self._debug_buf.data_ptr(), int(n_tokens)))
         return self._debug_buf
 
     def set_profiling(self, enable: bool) -> None:

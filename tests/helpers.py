@@ -35,3 +35,36 @@ def compare_embeddings(got: torch.Tensor, want: torch.Tensor):
     max_abs = float((got - want).abs().max())
     cos = torch.nn.functional.cosine_similarity(got, want, dim=1)
     return max_abs, float(cos.min())
+
+
+def hf_bias_table(rel_bias: torch.Tensor, max_distance: int) -> torch.Tensor:
+    """[heads][2R+1] fp32 relative-bias table built with HF's own bucket function: entry d + R is
+    rel_bias[bucket(d)] for d = key - query (the layout the attention kernels consume)."""
+    from transformers.models.t5.modeling_t5 import T5Attention
+
+    d = torch.arange(-max_distance, max_distance + 1)
+    buckets = T5Attention._relative_position_bucket(d, bidirectional=True, num_buckets=rel_bias.shape[0],
+                                                    max_distance=max_distance)
+    return rel_bias.float()[buckets].t().contiguous()
+
+
+def attention_fp64(qkv: torch.Tensor, lens, n_heads: int, lut: torch.Tensor, max_distance: int, d_kv: int = 64):
+    """Plain T5 self-attention in float64, per packed sequence and head: softmax(q k^T + lut[clamp(key - query)]) v
+    (no 1/sqrt(d) scaling).  qkv [T, 3 * heads * d_kv] (q | k | v).  Returns (out, W |V|), both [T, heads * d_kv]."""
+    x = qkv.double()
+    lut = lut.to(device=qkv.device, dtype=torch.float64)
+    inner = n_heads * d_kv
+    o = torch.empty(x.shape[0], inner, dtype=torch.float64, device=x.device)
+    wv = torch.empty_like(o)
+    t0 = 0
+    for L in lens:
+        L = int(L)
+        seq = x[t0:t0 + L]
+        q, k, v = (seq[:, i * inner:(i + 1) * inner].reshape(L, n_heads, d_kv).transpose(0, 1) for i in range(3))
+        pos = torch.arange(L, device=x.device)
+        idx = (pos[None, :] - pos[:, None]).clamp(-max_distance, max_distance) + max_distance
+        w = torch.softmax(q @ k.transpose(1, 2) + lut[:, idx], dim=-1)
+        o[t0:t0 + L] = (w @ v).transpose(0, 1).reshape(L, inner)
+        wv[t0:t0 + L] = (w @ v.abs()).transpose(0, 1).reshape(L, inner)
+        t0 += L
+    return o, wv

@@ -65,6 +65,19 @@ def test_host_only_entry_points(rpx_lib):
     assert rpx_lib.rpx_encoder_workspace_bytes(None, 1000, 10) == 0
 
 
+def test_packed_bytes_rejects_a_bias_table_attention_cannot_hold(rpx_lib):
+    """A relative-position range whose bias table does not fit the attention kernel's shared memory is refused
+    when the encoder is sized, not on its first encode call: 1584 is the largest range that fits."""
+    def cfg(R):
+        return _native.T5Config(vocab_size=384, d_model=1472, d_kv=64, d_ff=3584, num_layers=2, num_heads=6,
+                                rel_buckets=32, rel_max_distance=R, ln_eps=1e-6)
+
+    assert rpx_lib.rpx_encoder_packed_bytes(C.byref(cfg(1584))) > 0
+    for R in (1585, 2048):
+        assert rpx_lib.rpx_encoder_packed_bytes(C.byref(cfg(R))) == 0
+        assert "rel_max_distance" in _native.last_error()
+
+
 def test_relative_bucket_matches_hf_golden(rpx_lib):
     g = json.loads((ROOT / "tests" / "golden" / "bucket_table.json").read_text())
     got = [rpx_lib.rpx_t5_relative_bucket(r, g["num_buckets"], g["max_distance"]) for r in g["relative_position"]]
